@@ -2,6 +2,7 @@
 """bench.py — CogView-base 4B hot path on B200 (BASELINE.json metric: tokens/sec, train + AR sample).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload sample|train|both]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -50,7 +51,15 @@ def parse():
                     help="development only: leave out the host-core baseline leg (the default run includes it)")
     ap.add_argument("--dropout", type=float, default=0.1,
                     help="embedding/attention/hidden dropout of the training workload (reference scripts: 0.1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step of each workload returned as DIR/<name>.npy "
+                         "(float32; large outputs as a fixed seeded sample), to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm only samples timings)")
+    return args
 
 
 def measured_traffic(kernel):
@@ -199,6 +208,7 @@ def launches():
 # ----------------------------------------------------------------------------------------------------
 def run_sample(args, cfg, world, rank, dev_index):
     from cogview_b200.generation import sampling
+    torch.manual_seed(rank)            # weights and the sampling draws: the same run for the same arguments
     model = build_model(cfg, cfg["max_sequence_length"], "cuda").eval()
     nb = args.batch
     tmpl_host = make_template(nb, args.gen_tokens, seed=rank).pin_memory()
@@ -220,6 +230,7 @@ def run_sample(args, cfg, world, rank, dev_index):
     tokens_per_step = nb * args.gen_tokens * world
     l0 = launches()
     ms_dev, clocks = timed(step_dev, args.steps, args.warmup, dev_index)
+    outputs = dict(sample_tokens=holder["out"]) if args.dump_outputs else {}
     graph_nodes = 0
     kv = model.transformer._kv
     if kv is not None and getattr(kv, "runner", None) is not None:
@@ -234,6 +245,7 @@ def run_sample(args, cfg, world, rank, dev_index):
                gpu_launches=int(n_launch / max(1, (args.steps + args.warmup))) * args.steps)
     res["roofline"] = sample_roofline(model, nb, res["ms_per_step"], args.gen_tokens)
     res["params"] = param_count(model)
+    res["outputs"] = outputs
     del model
     torch.cuda.empty_cache()
     return res
@@ -329,6 +341,7 @@ def run_train(args, cfg, world, rank, dev_index, steps, warmup):
     from cogview_b200 import mpu
     from cogview_b200.model import (PyTorchDistributedDataParallel, gpt2_get_params_for_weight_decay_optimization)
     from cogview_b200.optim import FusedAdamW
+    torch.manual_seed(100 + rank)      # weights and dropout masks: the same run for the same arguments
     model = build_model(cfg, 0, "cuda", dropout=args.dropout).train()
     groups = gpt2_get_params_for_weight_decay_optimization(model)
     for g in groups:
@@ -380,6 +393,14 @@ def run_train(args, cfg, world, rank, dev_index, steps, warmup):
     l0 = launches()
     ms_dev, clocks = timed(step_dev, steps, warmup, dev_index)
     n_launch = launches() - l0
+    outputs = {}
+    if args.dump_outputs:
+        # the step returns the loss and updates the weights in place (the end-to-end steps below update them again)
+        g = torch.Generator().manual_seed(0)
+        outputs["train_loss"] = last["loss"].detach().view(1)
+        outputs["train_weights_sample"] = torch.cat([
+            p.detach().reshape(-1)[torch.randint(0, p.numel(), (min(p.numel(), 4096),), generator=g).cuda()].float()
+            for p in model.parameters()])
     ms_e2e, _ = timed(step_e2e, steps, 1, dev_index)
     loss_val = float(last["loss"].item())
     assert loss_val == loss_val and loss_val < 20.0, "training loss is not finite"
@@ -405,6 +426,7 @@ def run_train(args, cfg, world, rank, dev_index, steps, warmup):
         from cogview_b200 import _lib
         _lib.lib().cv_set_reserved_sms(0)
     res["roofline"] = gemm_roofline(cfg, b * s)
+    res["outputs"] = outputs
     del net, model, opt
     torch.cuda.empty_cache()
     return res
@@ -476,6 +498,11 @@ def run_vqvae(args, world, rank, dev_index, steps, warmup):
     l0 = launches()
     ms_dev, clocks = timed(step_dev, steps, warmup, dev_index)
     n_launch = launches() - l0
+    outputs = {}
+    if args.dump_outputs:
+        rec = keep["rec"].reshape(-1)
+        idx = torch.randperm(rec.numel(), generator=torch.Generator().manual_seed(0))[:1 << 22].sort().values
+        outputs = dict(vqvae_codes=keep["codes"], vqvae_images_sample=rec[idx.cuda()])
     ms_e2e, _ = timed(step_e2e, steps, 1, dev_index)
     assert keep["codes"].shape == (B, 1024) and int(keep["codes"].max()) < 8192
     assert bool(torch.isfinite(keep["rec"]).all())
@@ -493,7 +520,8 @@ def run_vqvae(args, world, rank, dev_index, steps, warmup):
                            parallelism="dp%d (independent images per rank, no collective)" % world),
                roofline_step=dict(bound="tensor", achieved=achieved, peak=pk["tf_sust"], unit="TFLOP/s",
                                   frac=achieved / pk["tf_sust"], peak_source=pk["src"],
-                                  note="whole round trip (224.6 GFLOP/image algorithmic) vs sustained cuBLAS bf16 peak"))
+                                  note="whole round trip (224.6 GFLOP/image algorithmic) vs sustained cuBLAS bf16 peak"),
+               outputs=outputs)
     del model
     torch.cuda.empty_cache()
     return res
@@ -767,6 +795,14 @@ def cpu_baseline_train(cfg, budget_s=25.0):
 
 
 # ----------------------------------------------------------------------------------------------------
+def write_outputs(directory, outputs):
+    """One DIR/<name>.npy per output, as float32 (exact for the token ids and codes, which stay below 2**24)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def _compact(d, keys):
     return {k: d[k] for k in keys if k in d}
 
@@ -795,7 +831,7 @@ def main():
         vals, walls = [], []
         for _ in range(args.warmup and 1):
             cpu_baseline_sample(cfg, args.batch, args.gen_tokens, budget_s=8.0)
-        for _ in range(max(1, min(args.steps, 3))):
+        for _ in range(args.steps):
             ts = time.perf_counter()
             cb = cpu_baseline_sample(cfg, args.batch, args.gen_tokens, budget_s=15.0)
             walls.append(time.perf_counter() - ts)
@@ -825,15 +861,18 @@ def main():
         mpu.initialize_model_parallel(1)
 
     line = dict(base)
+    outputs = {}
     if args.workload in ("sample", "both", "all"):
         r = run_sample(args, cfg, world, rank, local_rank)
+        outputs.update(r.pop("outputs"))
         line.update(value=r["value"], ms_per_step=r["ms_per_step"], e2e=r["e2e"], clocks=r["clocks"],
                     gpu_launches=r["gpu_launches"], roofline=r["roofline"],
                     config=dict(workload=workload_name, global_batch=args.batch * world, seq_len=1089,
                                 parallelism="dp%d (independent sequences per rank, no collective)" % world,
                                 l2="each decode step streams 7.9 GB of weights (>> 126 MB L2)", params=r["params"]))
     if args.workload in ("vqvae", "all"):
-        v = run_vqvae(args, world, rank, local_rank, max(3, args.steps), max(3, args.warmup))
+        v = run_vqvae(args, world, rank, local_rank, args.steps, max(3, args.warmup))
+        outputs.update(v.pop("outputs"))
         if args.workload == "vqvae":
             line.update(metric="images/sec (VQ-VAE encode+quantise+decode, 256x256)", unit="images/s", value=v["value"],
                         ms_per_step=v["ms_per_step"], e2e=v["e2e"], clocks=v["clocks"], gpu_launches=v["gpu_launches"],
@@ -843,8 +882,9 @@ def main():
                                            frac_of_sustained_tensor_peak=v["roofline_step"]["frac"])
         line["vqvae"] = v
     if args.workload in ("train", "both", "all"):
-        tsteps = args.train_steps or max(3, args.steps)
+        tsteps = args.train_steps or args.steps
         t = run_train(args, cfg, world, rank, local_rank, tsteps, max(3, args.warmup))
+        outputs.update(t.pop("outputs"))
         if args.workload == "train":
             line.update(metric="tokens/sec (train) CogView-4B seq1089", value=t["value"], ms_per_step=t["ms_per_step"],
                         e2e=t["e2e"], clocks=t["clocks"], gpu_launches=t["gpu_launches"], roofline=t["roofline"],
@@ -858,6 +898,8 @@ def main():
                                            gemm_frac_of_burst_peak=t["roofline"]["frac"], loss=t["loss"],
                                            exposed_comm_ms=t.get("exposed_comm_ms"))
         line["train"] = t
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, outputs)
     if rank == 0 and (args.skip_cpu_baseline or world > 1):
         # the CPU baseline is reported at N = 1 only (--skip-cpu-baseline: development runs)
         line["cpu_baseline"] = None

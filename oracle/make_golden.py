@@ -2,7 +2,7 @@
 
   python oracle/make_golden.py
 
-1. Imports the UNMODIFIED reference (oracle/ref_harness.py) and runs it on the seeded inputs of
+1. Places the UNMODIFIED reference under oracle/_ref (oracle/build_ref.py), imports it (oracle/ref_harness.py) and runs it on the seeded inputs of
    oracle/recipes.py (SURVEY §8(d) config 1; VQ-VAE new_model()).
 2. Asserts the travelling restatement oracle/cogview_oracle.py reproduces the reference (fp32).
 3. Writes compact fixtures to tests/golden/ (outputs only — weights/inputs are regenerated from seeds).
@@ -19,10 +19,11 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
 
 from oracle import cogview_oracle as O  # noqa: E402
-from oracle import recipes, ref_harness  # noqa: E402
+from oracle import build_ref, recipes, ref_harness  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
 VOCAB_STRIDE = 97  # logits are stored on every 97th vocab column (+ arg-max / top-8 per position)
+SEP40_VOCAB_STRIDE = 8 * VOCAB_STRIDE  # the int-sep logits on a coarser sample keep gpt2_config1.npz under 1 MB
 
 
 def close(a, b, tol, what):
@@ -118,7 +119,8 @@ def gpt2_golden(ref):
         logits_argmax=logits.detach().argmax(-1).numpy(),
         logits_top8_val=top8.values.numpy(), logits_top8_idx=top8.indices.numpy(),
         losses=losses.detach().numpy(), loss=np.float32(loss.item()),
-        logits_sep40_strided=lg_sep.detach()[:, :, ::VOCAB_STRIDE].numpy(),
+        logits_sep40_strided=lg_sep.detach()[:, :, ::SEP40_VOCAB_STRIDE].numpy(),
+        sep40_vocab_stride=np.int64(SEP40_VOCAB_STRIDE),
         grad_names=np.array(list(ref_grads.keys())),
         grad_samples=np.stack([sample_grad(g)[0] for g in ref_grads.values()]),
         grad_norms=np.array([sample_grad(g)[1] for g in ref_grads.values()], dtype=np.float64),
@@ -220,6 +222,8 @@ def vqvae_golden_256(ref, n=17):
 def main():
     os.makedirs(GOLD, exist_ok=True)
     torch.set_num_threads(8)
+    if not build_ref.build():
+        raise SystemExit("make_golden: the reference is not available under oracle/_ref")
     ref = ref_harness.load()
     gpt2_golden(ref)
     attention_golden(ref)

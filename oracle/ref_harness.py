@@ -1,6 +1,6 @@
-"""TEST INFRASTRUCTURE — imports the UNMODIFIED reference modules on CPU: from /root/reference in the build
-container, from oracle/_ref (the same files, placed by oracle/build_ref.py) on the GPU box.  Used by bench.py's
-reference arm (cpu_baseline.kind = "reference") and by
+"""TEST INFRASTRUCTURE — imports the UNMODIFIED reference modules on CPU from oracle/_ref, where
+oracle/build_ref.py (run by build()) places them.  Used by bench.py's reference arm (cpu_baseline.kind =
+"reference") and by
 oracle/make_golden.py to (a) validate the travelling restatement oracle/cogview_oracle.py against the
 real reference and (b) generate the golden fixtures under tests/golden/.
 
@@ -20,10 +20,7 @@ import types
 
 import torch
 
-REFERENCE_ROOT = os.environ.get("COGVIEW_REFERENCE", "/root/reference")
-if not os.path.isdir(os.path.join(REFERENCE_ROOT, "mpu")):
-    # the GPU box: the unmodified module files placed by oracle/build_ref.py (git-ignored, shipped with the snapshot)
-    REFERENCE_ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
+REFERENCE_ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 _loaded = {}
 

@@ -150,8 +150,8 @@ def test_weight_decay_parameter_groups():
 
 
 def test_bench_reference_arm_prints_the_contract_line():
-    """`bench.py --impl reference` (the reference's own modules from oracle/_ref — or /root/reference — on the host
-    cores; the oracle port when neither exists) on the tiny configuration: one JSON line with the contract's keys,
+    """`bench.py --impl reference` (the reference's own modules from oracle/_ref on the host cores; the oracle port
+    when build() could not place them there) on the tiny configuration: one JSON line with the contract's keys,
     `impl = reference`, a `cpu_baseline` describing the run and a zero-copy `e2e`."""
     import json
     import os
@@ -170,7 +170,7 @@ def test_bench_reference_arm_prints_the_contract_line():
         assert k in d, k
     assert d["impl"] == "reference" and d["unit"] == "tokens/s" and d["higher_is_better"] is True
     assert d["value"] > 0 and d["cpu_baseline"]["value"] == d["value"] and d["cpu_baseline"]["kind"] in ("reference", "port")
-    ref_here = os.path.isdir(os.path.join(root, "oracle", "_ref", "mpu")) or os.path.isdir("/root/reference/mpu")
+    ref_here = os.path.isdir(os.path.join(root, "oracle", "_ref", "mpu"))
     assert d["cpu_baseline"]["kind"] == ("reference" if ref_here else "port")
     assert d["cpu_baseline"]["cores"] >= 1 and "workload" in d["config"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}

@@ -80,7 +80,7 @@ def test_int_sep_mask_form(data):
     with torch.no_grad():
         logits, *_ = m(data["tokens"].cuda(), data["pos"].cuda(), 40, None, None, 0)
     g = data["g"]
-    stride = int(g["vocab_stride"])
+    stride = int(g["sep40_vocab_stride"])
     scale = np.abs(g["logits_sep40_strided"]).max()
     assert np.abs(logits.float().cpu()[:, :, ::stride].numpy() - g["logits_sep40_strided"]).max() < 3e-2 * scale
 
