@@ -78,6 +78,9 @@ def _declare(lib):
         "cv_colsum_bf16": [P, L, P, P, I, I, P],
         "cv_attn_sparse_fwd": [P, L, L, P, L, L, P, L, L, P, P, L, L, P, P, I, I, I, I, I, I, I, P],
         "cv_attn_sparse_bwd": [P, L, L, P, L, L, P, L, L, P, P, P, P, P, P, I, I, I, I, I, I, I, P],
+        "cv_attn_sparse_dropout_fwd": [P, L, L, P, L, L, P, L, L, P, P, L, L, P, P, I, I, I, I, I, I, I, F, U64, U32, P,
+                                       P],
+        "cv_attn_sparse_dropout_bwd": [P, L, L, P, L, L, P, L, L, P, P, P, P, P, P, I, I, I, I, I, I, I, F, P, P],
         "cv_decode_step": [ctypes.POINTER(DecodeStepArgs), P],
         "cv_sample_topk": [P, L, I, I, F, I, ctypes.POINTER(c_int), I, U64, P, P, P, P, L, P, P, P, P, P, P],
     })
@@ -85,6 +88,8 @@ def _declare(lib):
     lib.cv_attn_sparse_workspace_bytes.restype = L
     lib.cv_attn_sparse_bwd_workspace_bytes.argtypes = [I, I, I, I, I]
     lib.cv_attn_sparse_bwd_workspace_bytes.restype = L
+    lib.cv_attn_sparse_drop_mask_words.argtypes = [I, I, I, I, I, I]
+    lib.cv_attn_sparse_drop_mask_words.restype = L
     lib.cv_decode_step_workspace_bytes.argtypes = [I, I]
     lib.cv_decode_step_workspace_bytes.restype = L
     lib.cv_layernorm_bwd_workspace_bytes.argtypes = [I, I]

@@ -42,8 +42,9 @@ struct BwdParams {
     const float* delta;  // [b, heads, s]
     float* dq_acc;       // [b, s, heads*HD] fp32, zero-initialised
     __nv_bfloat16* dqkv; // [b, s, 3*heads*HD]
-    const uint32_t* drop_mask;  // keep bits written by the forward, key-major ([b, heads, nkb*128, nqb, 4]: the 128 query
+    const uint32_t* drop_mask;  // keep bits written by the forward, key-major ([b, heads, keep_rows, nqb, 4]: the 128 query
                                 // bits of (key, query block) are one 16-byte load for the thread that owns the key) or null
+    int keep_rows;              // key rows per (batch, head) of drop_mask: nqb*128 (dense, band pass), npt*128 (pivot pass)
     float drop_scale;           // 1 / (1 - p)
     // sparse training attention (mpu/sparse_transformer.py:675-725), two launches that share lse / delta / dq_acc:
     //   MODE_BAND : keys = the sequence, key j visible to query i iff band_start(i) <= j <= i
@@ -206,7 +207,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         const float masked_val = -10000.0f * LOG2E;
         const int my_pos = (MODE == MODE_PIVOT) ? (kj < p.sk ? p.piv_pos[(size_t)batch * p.sk + kj] : 0x7fffffff) : 0;
         const size_t stat_base = ((size_t)batch * p.heads + head) * p.s;
-        const size_t keep_base = ((size_t)batch * p.heads + head) * (size_t)nqb * BLK;   // key rows are padded to blocks
+        const size_t keep_base = ((size_t)batch * p.heads + head) * (size_t)p.keep_rows;   // key rows padded to blocks
         int stage = 0;
         float pre_lse, pre_delta;
         uint4 pre_keep = make_uint4(0, 0, 0, 0);
@@ -475,6 +476,7 @@ extern "C" int cv_attn_bwd(const void* q, int64_t ldq, int64_t bsq, const void* 
     p.lse = lse; p.delta = delta; p.dq_acc = dq_acc;
     p.dqkv = static_cast<__nv_bfloat16*>(dqkv);
     p.drop_mask = dropout_p > 0.f ? drop_mask : nullptr;
+    p.keep_rows = (s + BLK - 1) / BLK * BLK;
     p.drop_scale = dropout_p > 0.f ? 1.0f / (1.0f - dropout_p) : 1.0f;
     p.sk = s; p.kv_rows = s; p.sp_w = 1; p.sp_times = 1; p.piv_pos = nullptr; p.piv_bias_log2 = 0.f;
     static bool attr_set = false;
@@ -546,6 +548,18 @@ extern "C" int cv_attn_sparse_bwd(const void* q, int64_t ldq, int64_t bsq, const
                                   const void* d_out, const float* lse, void* dqkv, void* workspace, int b, int heads,
                                   int head_dim, int s, int n_piv, int query_window, int key_window_times,
                                   void* stream) {
+    return cv_attn_sparse_dropout_bwd(q, ldq, bsq, k, ldk, bsk, v, ldv, bsv, pivot_idx, out, d_out, lse, dqkv, workspace,
+                                      b, heads, head_dim, s, n_piv, query_window, key_window_times, 0.f, nullptr, stream);
+}
+
+extern "C" int cv_attn_sparse_dropout_bwd(const void* q, int64_t ldq, int64_t bsq, const void* k, int64_t ldk,
+                                          int64_t bsk, const void* v, int64_t ldv, int64_t bsv,
+                                          const int64_t* pivot_idx, const void* out, const void* d_out,
+                                          const float* lse, void* dqkv, void* workspace, int b, int heads,
+                                          int head_dim, int s, int n_piv, int query_window, int key_window_times,
+                                          float dropout_p, const uint32_t* drop_mask, void* stream) {
+    CV_REQUIRE(dropout_p >= 0.f && dropout_p < 1.f, "dropout probability must be in [0, 1)");
+    CV_REQUIRE(dropout_p == 0.f || drop_mask != nullptr, "attention dropout needs the keep mask saved by the forward");
     CV_REQUIRE(q && k && v && pivot_idx && out && d_out && lse && dqkv && workspace, "null pointer");
     CV_REQUIRE(head_dim == HD, "head_dim must be 64");
     CV_REQUIRE(b > 0 && heads > 0 && s > 0 && n_piv > 0 && n_piv <= s, "bad sizes");
@@ -591,7 +605,12 @@ extern "C" int cv_attn_sparse_bwd(const void* q, int64_t ldq, int64_t bsq, const
     p.scale = 1.0f / sqrtf((float)head_dim);
     p.scale_log2 = p.scale * LOG2E;
     p.lse = lse; p.delta = delta; p.dq_acc = dq_acc;
-    p.drop_mask = nullptr; p.drop_scale = 1.0f;
+    // keep bits (cv_attn_sparse_drop_mask_words): band pass reads region [0], pivot pass region [1]
+    const int nqb = (s + BLK - 1) / BLK, npt = (n_piv + BLK - 1) / BLK;
+    const uint32_t* band_keep = dropout_p > 0.f ? drop_mask : nullptr;
+    const uint32_t* piv_keep = dropout_p > 0.f ? drop_mask + (size_t)b * heads * nqb * BLK * nqb * 4 : nullptr;
+    p.drop_mask = band_keep; p.keep_rows = nqb * BLK;
+    p.drop_scale = dropout_p > 0.f ? 1.0f / (1.0f - dropout_p) : 1.0f;
     p.sp_w = query_window; p.sp_times = key_window_times;
     p.piv_bias_log2 = logf((float)(s / n_piv)) * LOG2E;
     static bool attr_set = false;
@@ -608,6 +627,7 @@ extern "C" int cv_attn_sparse_bwd(const void* q, int64_t ldq, int64_t bsq, const
     if (key_window_times * query_window < s) {       // some query sees pivots at all
         p.dqkv = dpiv;
         p.sk = n_piv; p.kv_rows = n_piv; p.piv_pos = pos32;
+        p.drop_mask = piv_keep; p.keep_rows = npt * BLK;
         attn_bwd_kernel<MODE_PIVOT><<<dim3((n_piv + BLK - 1) / BLK, heads, b), NUM_THREADS, SMEM_BYTES, st>>>(
             tmQ, tmPK, tmPV, tmDO, p);
         CV_LAUNCH_CHECK();

@@ -60,11 +60,46 @@ struct AttnParams {
     int sp_w, sp_times, n_piv;
     const int* piv_pos;     // [b, n_piv] positions of the gathered pivot keys
     float piv_bias_log2;    // log(s / n_piv) * log2(e)
+    // sparse with dropout: drop_mask holds the three regions of SparseKeepLayout instead of the two above
+    int sp_npt;             // ceil(n_piv / 128): pivot tiles
+    int sp_tiles;           // longest tile list of any query block (row length of the query-major region)
+    const uint2* keep_q;    // start of that query-major region, as pairs of words (one 64-key half of a tile)
 };
 
-__device__ __forceinline__ int band_start(int i, int w, int times) {
+__host__ __device__ __forceinline__ int band_start(int i, int w, int times) {
     const int g = i / w - times + 1;
     return g > 0 ? g * w : 0;
+}
+
+// Tile list of query block qb in sparse mode: band tiles jb0 .. jb0 + nband - 1 of the real keys, then npt pivot tiles
+// (all of them if any query of the block can see a pivot at all, else none).  Shared by the attention kernel, the
+// keep-bit generator and the host, so all three walk the same list.
+struct SparseTiles { int jb0, nband, npt; };
+__host__ __device__ __forceinline__ SparseTiles sparse_tiles(int qb, int s, int w, int times, int n_piv) {
+    const int q0 = qb * BQ;
+    const int q_last = (q0 + BQ < s ? q0 + BQ : s) - 1;
+    SparseTiles t;
+    t.jb0 = band_start(q0, w, times) / BKV;
+    t.nband = q_last / BKV - t.jb0 + 1;
+    t.npt = band_start(q_last, w, times) > 0 ? (n_piv + BKV - 1) / BKV : 0;
+    return t;
+}
+
+// Keep bits of the sparse attention-probability dropout (cv_attn_sparse_drop_mask_words), uint32 words:
+//   [0] band key-major  at 0:        [b, heads, nqb*128 (key), nqb, 4]  — the dense key-major layout (s = sq = sk)
+//   [1] pivot key-major at piv_off:  [b, heads, npt*128 (pivot slot), nqb, 4]
+//   [2] query-major     at qmaj_off: [b, heads, nqb*128 (query), tiles, 4], indexed by the tile-list position j
+//       (band tiles first, then pivot tiles), so the attention kernel walks it linearly
+// bit i of word w of a key-major (key, query block qb) entry is query qb*128 + 32w + i; bit i of word w of a
+// query-major (query, j) entry is key 32w + i of tile j.  Tiles outside a query block's list stay unwritten.
+struct SparseKeepLayout { size_t piv_off, qmaj_off, words; };
+__host__ __device__ __forceinline__ SparseKeepLayout sparse_keep_layout(int b, int heads, int nqb, int npt, int tiles) {
+    const size_t bh = (size_t)b * heads, key_row = (size_t)nqb * 4;   // words per key row
+    SparseKeepLayout l;
+    l.piv_off = bh * nqb * BKV * key_row;
+    l.qmaj_off = l.piv_off + bh * npt * BKV * key_row;
+    l.words = l.qmaj_off + bh * nqb * BQ * (size_t)tiles * 4;
+    return l;
 }
 
 template <bool DROPOUT, bool SPARSE>
@@ -102,11 +137,10 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
     // block can see a pivot at all); one tile list for the three roles
     int jb0 = 0, nband = nkb;
     if (SPARSE) {
-        const int q_last = min(q0 + BQ, p.sq) - 1;
-        jb0 = band_start(q0, p.sp_w, p.sp_times) / BKV;
-        nband = q_last / BKV - jb0 + 1;
-        const int npt = band_start(q_last, p.sp_w, p.sp_times) > 0 ? (p.n_piv + BKV - 1) / BKV : 0;
-        nkb = nband + npt;
+        const SparseTiles st = sparse_tiles(qb, p.sq, p.sp_w, p.sp_times, p.n_piv);
+        jb0 = st.jb0;
+        nband = st.nband;
+        nkb = nband + st.npt;
     }
 
     if (warp_idx == 0 && lane == 0) {
@@ -209,7 +243,14 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         const float masked_val = -10000.0f * LOG2E;
         const uint4* keep_row = nullptr;
         uint4 pre_keep = make_uint4(0u, 0u, 0u, 0u);
-        if (DROPOUT) {
+        uint32_t keep_off = 0u;
+        if (DROPOUT && SPARSE) {
+            // query-major region (p.keep_q): one row of sp_tiles entries per query, in tile-list order.  This thread
+            // reads only its half's two words, after the scores are in registers (the row-maximum exchange covers the
+            // load), and holds a 32-bit row offset instead of a pointer: the sparse tile walk is at the register limit
+            // (168) even without dropout
+            keep_off = (uint32_t)((((uint32_t)batch * p.heads + head) * p.nqb_all * BQ + qi) * p.sp_tiles * 2 + hf);
+        } else if (DROPOUT) {
             const size_t region = (size_t)p.b * p.heads * p.nkb_all * p.nqb_all * (BQ * 4);   // words per region
             keep_row = reinterpret_cast<const uint4*>(p.drop_mask + region) +
                        (((size_t)batch * p.heads + head) * p.nqb_all * BQ + qi) * p.nkb_all;
@@ -218,7 +259,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
 
         for (int j = 0; j < nkb; ++j) {
             uint32_t kw0 = 0u, kw1 = 0u;                // keep bits of this row over this thread's 64 keys
-            if (DROPOUT) {
+            if (DROPOUT && !SPARSE) {
                 kw0 = hf ? pre_keep.z : pre_keep.x;
                 kw1 = hf ? pre_keep.w : pre_keep.y;
                 if (j + 1 < nkb) pre_keep = keep_row[j + 1];
@@ -270,6 +311,11 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
                     mx = fmaxf(mx, v);
                 }
             }
+            if (DROPOUT && SPARSE) {
+                const uint2 kw = p.keep_q[keep_off + j * 2];
+                kw0 = kw.x;
+                kw1 = kw.y;
+            }
             // row maximum over both halves
             sX[((j & 1) * 2 + hf) * BQ + row] = mx;
             named_bar_sync(3 + q, 64);
@@ -290,8 +336,14 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
                 const __nv_bfloat162* pb = reinterpret_cast<const __nv_bfloat162*>(&pk);
 #pragma unroll
                 for (int t = 0; t < 4; ++t) psum += __low2float(pb[t]) + __high2float(pb[t]);
-                if (DROPOUT) {   // dropout acts on the normalised probabilities: the row sum stays undropped; the
-                                 // 1/(1-p) scale is applied once to the output row at the end
+                if (DROPOUT && SPARSE) {   // as below, on the packed words (bf16 zero = 0x0000): e[] is dead here
+                    const uint32_t w = ((c >> 2) == 0 ? kw0 : kw1) >> ((c & 3) * 8);
+                    pk.x &= ((w & 1u) ? 0x0000FFFFu : 0u) | ((w & 2u) ? 0xFFFF0000u : 0u);
+                    pk.y &= ((w & 4u) ? 0x0000FFFFu : 0u) | ((w & 8u) ? 0xFFFF0000u : 0u);
+                    pk.z &= ((w & 16u) ? 0x0000FFFFu : 0u) | ((w & 32u) ? 0xFFFF0000u : 0u);
+                    pk.w &= ((w & 64u) ? 0x0000FFFFu : 0u) | ((w & 128u) ? 0xFFFF0000u : 0u);
+                } else if (DROPOUT) {   // dropout acts on the normalised probabilities: the row sum stays undropped;
+                                        // the 1/(1-p) scale is applied once to the output row at the end
                     const uint32_t w = (c >> 2) == 0 ? kw0 : kw1;
 #pragma unroll
                     for (int t = 0; t < 8; ++t) e[t] = ((w >> ((c & 3) * 8 + t)) & 1u) ? e[t] : 0.f;
@@ -358,18 +410,31 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
 // ahead of the attention kernel at full occupancy (inside the attention kernel the same work sits on the softmax
 // warps' critical path: measured +200 us per call at the 4B shape).  One thread per (query row, key tile): a
 // Philox4x32-10 call seeds four 32-step LCG streams, keep iff state >= p * 2^32.  Writes both layouts (AttnParams).
-__global__ void __launch_bounds__(128, 4)
+// SPARSE: blockIdx.y is the position j in the block's tile list (sparse_tiles) and the three regions of
+// SparseKeepLayout are written.  A band tile keeps its key-tile index as counter, pivot tile t counts as key tile
+// nkb_all + t: the pivot slots and the band keys of one query draw from disjoint counters.  Either way every decision
+// is a pure function of (seed, site, batch, head, query, key or pivot slot), which checkpoint recomputation relies on.
+template <bool SPARSE>
+__global__ void __launch_bounds__(128, SPARSE ? 3 : 4)   // sparse: a few more live values; 3 blocks / SM keep it spill-free
 attn_dropout_mask_kernel(const AttnParams p) {
     const int qb = blockIdx.x, j = blockIdx.y;
     const int head = blockIdx.z % p.heads, batch = blockIdx.z / p.heads;
     const int q0 = qb * BQ;
-    int kmax = q0 + BQ + p.off;
-    if (kmax < p.sep_eff) kmax = p.sep_eff;
-    if (kmax > p.sk) kmax = p.sk;
-    if (j * BKV >= kmax) return;                 // tile never visited by the attention kernels
+    int ctile = j;                               // counter tile: the key tile, or nkb_all + pivot tile
+    if (SPARSE) {
+        const SparseTiles st = sparse_tiles(qb, p.sq, p.sp_w, p.sp_times, p.n_piv);
+        if (j >= st.nband + st.npt) return;      // beyond this block's tile list
+        ctile = j < st.nband ? st.jb0 + j : p.nkb_all + (j - st.nband);
+    } else {
+        int kmax = q0 + BQ + p.off;
+        if (kmax < p.sep_eff) kmax = p.sep_eff;
+        if (kmax > p.sk) kmax = p.sk;
+        if (j * BKV >= kmax) return;             // tile never visited by the attention kernels
+    }
     const int lane = threadIdx.x & 31, wq = threadIdx.x >> 5;
     const int qi = q0 + threadIdx.x;
-    const uint64_t ctr = (((uint64_t)batch * p.heads + head) * p.sq + qi) * p.nkb_all + j;
+    const int ctr_tiles = SPARSE ? p.nkb_all + p.sp_npt : p.nkb_all;
+    const uint64_t ctr = (((uint64_t)batch * p.heads + head) * p.sq + qi) * ctr_tiles + ctile;
     const uint4 r0 = philox4x32_10(p.drop.seed, ctr, p.drop.stream);
     uint32_t rng[4] = {r0.x, r0.y, r0.z, r0.w};
     uint32_t wrow[4], wkey[4];
@@ -388,10 +453,21 @@ attn_dropout_mask_kernel(const AttnParams p) {
         wkey[g] = mine;
     }
     const size_t bh = (size_t)batch * p.heads + head;
-    const size_t region = (size_t)p.b * p.heads * p.nkb_all * p.nqb_all * (BQ * 4);
-    reinterpret_cast<uint4*>(p.drop_mask + region)[(bh * p.nqb_all * BQ + qi) * p.nkb_all + j] =
-        make_uint4(wrow[0], wrow[1], wrow[2], wrow[3]);
-    uint32_t* dm = p.drop_mask + ((bh * p.nkb_all * BKV + j * BKV + lane) * p.nqb_all + qb) * 4 + wq;
+    uint32_t* dm;
+    if (SPARSE) {
+        const SparseKeepLayout l = sparse_keep_layout(p.b, p.heads, p.nqb_all, p.sp_npt, p.sp_tiles);
+        reinterpret_cast<uint4*>(p.drop_mask + l.qmaj_off)[(bh * p.nqb_all * BQ + qi) * p.sp_tiles + j] =
+            make_uint4(wrow[0], wrow[1], wrow[2], wrow[3]);
+        dm = ctile < p.nkb_all
+                 ? p.drop_mask + ((bh * p.nkb_all * BKV + ctile * BKV + lane) * p.nqb_all + qb) * 4 + wq
+                 : p.drop_mask + l.piv_off +
+                       ((bh * p.sp_npt * BKV + (ctile - p.nkb_all) * BKV + lane) * p.nqb_all + qb) * 4 + wq;
+    } else {
+        const size_t region = (size_t)p.b * p.heads * p.nkb_all * p.nqb_all * (BQ * 4);
+        reinterpret_cast<uint4*>(p.drop_mask + region)[(bh * p.nqb_all * BQ + qi) * p.nkb_all + j] =
+            make_uint4(wrow[0], wrow[1], wrow[2], wrow[3]);
+        dm = p.drop_mask + ((bh * p.nkb_all * BKV + j * BKV + lane) * p.nqb_all + qb) * 4 + wq;
+    }
 #pragma unroll
     for (int g = 0; g < 4; ++g) dm[(size_t)g * 32 * p.nqb_all * 4] = wkey[g];
 }
@@ -444,6 +520,7 @@ extern "C" int cv_attn_fwd(const void* q, int64_t ldq, int64_t bsq, const void* 
         p.nqb_all = (sq + BQ - 1) / BQ;
     }
     p.sp_w = 0; p.sp_times = 0; p.n_piv = 0; p.piv_pos = nullptr; p.piv_bias_log2 = 0.f;
+    p.sp_npt = 0; p.sp_tiles = 0; p.keep_q = nullptr;
     static bool attr_set = false;
     if (!attr_set) {
         CV_CUDA(cudaFuncSetAttribute(attn_fwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
@@ -452,7 +529,7 @@ extern "C" int cv_attn_fwd(const void* q, int64_t ldq, int64_t bsq, const void* 
     }
     dim3 grid((sq + BQ - 1) / BQ, heads, b);
     if (dropout_p > 0.f) {
-        attn_dropout_mask_kernel<<<dim3(p.nqb_all, p.nkb_all, b * heads), 128, 0, s>>>(p);
+        attn_dropout_mask_kernel<false><<<dim3(p.nqb_all, p.nkb_all, b * heads), 128, 0, s>>>(p);
         CV_LAUNCH_CHECK();
         attn_fwd_kernel<true, false><<<grid, NUM_THREADS, SMEM_BYTES, s>>>(tmQ, tmK, tmV, tmK, tmV, p);
     }
@@ -482,6 +559,16 @@ __global__ void gather_pivots_kernel(const __nv_bfloat16* __restrict__ k, int64_
         d[h / 8 + i] = vs[i];
     }
 }
+
+// longest sparse tile list over the query blocks (row length of the query-major keep-bit region)
+int sparse_max_tiles(int s, int w, int times, int n_piv) {
+    int m = 0;
+    for (int qb = 0; qb < (s + BQ - 1) / BQ; ++qb) {
+        const SparseTiles t = sparse_tiles(qb, s, w, times, n_piv);
+        m = std::max(m, t.nband + t.npt);
+    }
+    return m;
+}
 }  // namespace
 
 extern "C" int64_t cv_attn_sparse_workspace_bytes(int b, int heads, int head_dim, int n_piv) {
@@ -489,11 +576,32 @@ extern "C" int64_t cv_attn_sparse_workspace_bytes(int b, int heads, int head_dim
     return ((int64_t)b * n_piv * 2 * h * 2 + 255) / 256 * 256 + (int64_t)b * n_piv * 4;
 }
 
+extern "C" int64_t cv_attn_sparse_drop_mask_words(int b, int heads, int s, int n_piv, int query_window,
+                                                  int key_window_times) {
+    if (b <= 0 || heads <= 0 || s <= 0 || n_piv <= 0 || query_window <= 0 || key_window_times <= 0) return 0;
+    const int nqb = (s + BQ - 1) / BQ, npt = (n_piv + BKV - 1) / BKV;
+    return (int64_t)sparse_keep_layout(b, heads, nqb, npt, sparse_max_tiles(s, query_window, key_window_times, n_piv))
+        .words;
+}
+
 extern "C" int cv_attn_sparse_fwd(const void* q, int64_t ldq, int64_t bsq, const void* k, int64_t ldk, int64_t bsk,
                                   const void* v, int64_t ldv, int64_t bsv, const int64_t* pivot_idx, void* out,
                                   int64_t ldo, int64_t bso, float* lse, void* workspace, int b, int heads,
                                   int head_dim, int s, int n_piv, int query_window, int key_window_times,
                                   void* stream) {
+    return cv_attn_sparse_dropout_fwd(q, ldq, bsq, k, ldk, bsk, v, ldv, bsv, pivot_idx, out, ldo, bso, lse, workspace, b,
+                                      heads, head_dim, s, n_piv, query_window, key_window_times, 0.f, 0, 0, nullptr,
+                                      stream);
+}
+
+extern "C" int cv_attn_sparse_dropout_fwd(const void* q, int64_t ldq, int64_t bsq, const void* k, int64_t ldk,
+                                          int64_t bsk, const void* v, int64_t ldv, int64_t bsv,
+                                          const int64_t* pivot_idx, void* out, int64_t ldo, int64_t bso, float* lse,
+                                          void* workspace, int b, int heads, int head_dim, int s, int n_piv,
+                                          int query_window, int key_window_times, float dropout_p, uint64_t seed,
+                                          uint32_t site, uint32_t* drop_mask, void* stream) {
+    CV_REQUIRE(dropout_p >= 0.f && dropout_p < 1.f, "dropout probability must be in [0, 1)");
+    CV_REQUIRE(dropout_p == 0.f || drop_mask != nullptr, "attention dropout needs the keep-mask buffer");
     CV_REQUIRE(q && k && v && pivot_idx && out && workspace, "null pointer");
     CV_REQUIRE(head_dim == HD, "head_dim must be 64 (CogView: hidden / heads = 64)");
     CV_REQUIRE(b > 0 && heads > 0 && s > 0 && n_piv > 0 && n_piv <= s, "bad sizes");
@@ -529,13 +637,37 @@ extern "C" int cv_attn_sparse_fwd(const void* q, int64_t ldq, int64_t bsq, const
     p.nqb_all = (s + BQ - 1) / BQ;
     p.sp_w = query_window; p.sp_times = key_window_times; p.n_piv = n_piv; p.piv_pos = pos32;
     p.piv_bias_log2 = logf((float)(s / n_piv)) * LOG2E;           // integer division as in :697
-    static bool attr_set = false;
-    if (!attr_set) {
-        CV_CUDA(cudaFuncSetAttribute(attn_fwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        attr_set = true;
-    }
+    p.sp_npt = (n_piv + BKV - 1) / BKV;
+    p.sp_tiles = 0; p.keep_q = nullptr;
     dim3 grid((s + BQ - 1) / BQ, heads, b);
-    attn_fwd_kernel<false, true><<<grid, NUM_THREADS, SMEM_BYTES, st>>>(tmQ, tmK, tmV, tmPK, tmPV, p);
+    if (dropout_p > 0.f) {
+        static bool attr_set_drop = false;
+        if (!attr_set_drop) {
+            CV_CUDA(cudaFuncSetAttribute(attn_fwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         SMEM_BYTES));
+            attr_set_drop = true;
+        }
+        const cvh::HostDropout hd = cvh::make_dropout(dropout_p, seed, site);
+        p.drop.p = hd.p; p.drop.scale = hd.scale; p.drop.threshold = hd.threshold; p.drop.stream = hd.stream;
+        p.drop.seed = hd.seed;
+        p.drop_mask = drop_mask;
+        p.sp_tiles = sparse_max_tiles(s, query_window, key_window_times, n_piv);
+        CV_REQUIRE((int64_t)b * heads * p.nqb_all * BQ * p.sp_tiles * 2 < (int64_t(1) << 32),
+                   "batch x heads x sequence too large for the sparse attention keep bits");
+        p.keep_q = reinterpret_cast<const uint2*>(
+            drop_mask + sparse_keep_layout(b, heads, p.nqb_all, p.sp_npt, p.sp_tiles).qmaj_off);
+        attn_dropout_mask_kernel<true><<<dim3(p.nqb_all, p.sp_tiles, b * heads), 128, 0, st>>>(p);
+        CV_LAUNCH_CHECK();
+        attn_fwd_kernel<true, true><<<grid, NUM_THREADS, SMEM_BYTES, st>>>(tmQ, tmK, tmV, tmPK, tmPV, p);
+    } else {
+        static bool attr_set = false;
+        if (!attr_set) {
+            CV_CUDA(cudaFuncSetAttribute(attn_fwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         SMEM_BYTES));
+            attr_set = true;
+        }
+        attn_fwd_kernel<false, true><<<grid, NUM_THREADS, SMEM_BYTES, st>>>(tmQ, tmK, tmV, tmPK, tmPV, p);
+    }
     CV_LAUNCH_CHECK();
     return 0;
 }

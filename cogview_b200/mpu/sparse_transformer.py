@@ -157,12 +157,6 @@ class SparseSpec:
         self.times = int(key_window_times)
 
 
-def _no_sparse_dropout(drops):
-    if drops is not None and drops['attn'][0] > 0:
-        raise NotImplementedError('attention-probability dropout is not available with sparse training attention '
-                                  '(is_sparse=1): set attention_dropout_prob = 0')
-
-
 def layer_forward(x, am_x, P, heads, eps, b, sq, sep, kv=None, save=None, attn=None, drops=None):
     """One Sandwich-LN block (mpu/sparse_transformer.py:314-342) on the fp32 residual stream x [b*sq, h].
 
@@ -183,11 +177,17 @@ def layer_forward(x, am_x, P, heads, eps, b, sq, sep, kv=None, save=None, attn=N
     if attn is not None:            # sparse inference: attention over a gathered key set
         ctx, lse = attn(q), None
     elif isinstance(sep, SparseSpec):   # sparse training: causal band + gathered pivots, one softmax
-        _no_sparse_dropout(drops)
-        if training:
-            ctx, lse = ops.attn_sparse_fwd(q, k, v, heads, sep.pivot_idx, sep.w, sep.times, want_lse=True)
+        sp = (q, k, v, heads, sep.pivot_idx, sep.w, sep.times)
+        if training and drops is not None and drops['attn'][0] > 0:
+            ctx, lse, amask = ops.attn_sparse_fwd(*sp, want_lse=True, dropout=drops['attn'])
+            drops['attn_mask'] = amask
+        elif training:
+            ctx, lse = ops.attn_sparse_fwd(*sp, want_lse=True)
+        elif drops is not None and drops['attn'][0] > 0:   # forward only (checkpointed pass): same site, mask not kept
+            ctx, _ = ops.attn_sparse_fwd(*sp, dropout=drops['attn'])
+            lse = None
         else:
-            ctx, lse = ops.attn_sparse_fwd(q, k, v, heads, sep.pivot_idx, sep.w, sep.times), None
+            ctx, lse = ops.attn_sparse_fwd(*sp), None
     elif training and drops is not None and drops['attn'][0] > 0:
         ctx, lse, amask = ops.attn_fwd(q, k, v, heads, sep=sep, want_lse=True, dropout=drops['attn'])
         drops['attn_mask'] = amask
@@ -249,7 +249,8 @@ def layer_backward(d_out, saved, P, heads, b, sq, sep, drops=None):
     use_ad = bool(drops) and drops['attn'][0] > 0
     if isinstance(sep, SparseSpec):
         d_qkv = ops.attn_sparse_bwd(qkv3[..., :h], qkv3[..., h:2 * h], qkv3[..., 2 * h:], ctx, d_ctx.view(b, sq, h), lse,
-                                    heads, sep.pivot_idx, sep.w, sep.times)
+                                    heads, sep.pivot_idx, sep.w, sep.times, dropout_p=drops['attn'][0] if use_ad else 0.0,
+                                    drop_mask=drops['attn_mask'] if use_ad else None)
     else:
         d_qkv = ops.attn_bwd(qkv3[..., :h], qkv3[..., h:2 * h], qkv3[..., 2 * h:], ctx, d_ctx.view(b, sq, h), lse, heads,
                              sep=sep, dropout_p=drops['attn'][0] if use_ad else 0.0,
@@ -347,29 +348,39 @@ class GPT2ParallelSelfAttention(torch.nn.Module):
 
 
 class _AttnFn(torch.autograd.Function):
+    """dropout: None or (p, seed, site) of the attention-probability dropout (sparse mode only)."""
+
     @staticmethod
-    def forward(ctx, q, k, v, heads, sep):
-        if isinstance(sep, SparseSpec):
+    def forward(ctx, q, k, v, heads, sep, dropout=None):
+        mask = None
+        if isinstance(sep, SparseSpec) and dropout is not None:
+            out, lse, mask = ops.attn_sparse_fwd(q, k, v, heads, sep.pivot_idx, sep.w, sep.times, want_lse=True,
+                                                 dropout=dropout)
+        elif isinstance(sep, SparseSpec):
             out, lse = ops.attn_sparse_fwd(q, k, v, heads, sep.pivot_idx, sep.w, sep.times, want_lse=True)
         else:
             out, lse = ops.attn_fwd(q, k, v, heads, sep=sep, want_lse=True)
-        ctx.save_for_backward(q, k, v, out, lse)
-        ctx.cfg = (heads, sep)
+        if mask is not None:
+            ctx.save_for_backward(q, k, v, out, lse, mask)
+        else:
+            ctx.save_for_backward(q, k, v, out, lse)
+        ctx.cfg = (heads, sep, dropout[0] if mask is not None else 0.0)
         return out
 
     @staticmethod
     def backward(ctx, d_out):
-        q, k, v, out, lse = ctx.saved_tensors
-        heads, sep = ctx.cfg
+        q, k, v, out, lse = ctx.saved_tensors[:5]
+        heads, sep, p_drop = ctx.cfg
         if q.shape[1] != k.shape[1]:
             raise NotImplementedError('attention backward with memory (sq != sk) is not supported')
         if isinstance(sep, SparseSpec):
             d_qkv = ops.attn_sparse_bwd(q, k, v, out, _as_bf16(d_out).contiguous(), lse, heads, sep.pivot_idx, sep.w,
-                                        sep.times)
+                                        sep.times, dropout_p=p_drop,
+                                        drop_mask=ctx.saved_tensors[5] if p_drop > 0 else None)
         else:
             d_qkv = ops.attn_bwd(q, k, v, out, _as_bf16(d_out).contiguous(), lse, heads, sep=sep)
         h = q.shape[2]
-        return d_qkv[..., :h], d_qkv[..., h:2 * h], d_qkv[..., 2 * h:], None, None
+        return d_qkv[..., :h], d_qkv[..., h:2 * h], d_qkv[..., 2 * h:], None, None, None
 
 
 @torch.jit.ignore
@@ -719,15 +730,19 @@ def sparse_attention(q, k, v, pivot_idx, pivot_attention_mask=None, query_window
     """mpu/sparse_transformer.py:675-725 on [b, np, s, hn] tensors (API parity; the model path reads the packed QKV
     GEMM output in place).  `pivot_attention_mask` is accepted for signature parity: the kernel evaluates the mask the
     reference builds (rmask of :491-496 gathered at pivot_idx, :569) in closed form — pivot p is visible to query i
-    iff pivot_idx[p] < band_start(i)."""
-    if attention_dropout is not None and attention_dropout.training and attention_dropout.p > 0:
-        raise NotImplementedError('attention-probability dropout is not available with sparse training attention')
+    iff pivot_idx[p] < band_start(i).  An `attention_dropout` module in training mode applies its p to the joint
+    softmax inside the kernel (counter-based keep bits, seed drawn from torch's generator as in standard_attention;
+    the reference draws from the model-parallel RNG tracker, :719-721).  Differentiable."""
     b, nh, s, hn = q.shape
 
     def tok_major(t):
         return _as_bf16(t).permute(0, 2, 1, 3).reshape(b, t.shape[2], nh * hn).contiguous()
 
-    ctx = _AttnFn.apply(tok_major(q), tok_major(k), tok_major(v), nh, SparseSpec(pivot_idx, query_window, key_window_times))
+    drop = None
+    if attention_dropout is not None and attention_dropout.training and attention_dropout.p > 0:
+        drop = (float(attention_dropout.p), int(torch.randint(0, 2 ** 62, (1,)).item()), 0)
+    ctx = _AttnFn.apply(tok_major(q), tok_major(k), tok_major(v), nh, SparseSpec(pivot_idx, query_window, key_window_times),
+                        drop)
     return ctx.view(b, s, nh, hn).permute(0, 2, 1, 3).to(q.dtype)
 
 

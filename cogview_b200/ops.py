@@ -176,9 +176,10 @@ def attn_bwd(q, k, v, out, d_out, lse, heads, *, sep=0, dropout_p=0.0, drop_mask
     return dqkv
 
 
-def attn_sparse_fwd(q, k, v, heads, pivot_idx, query_window, key_window_times, *, want_lse=False):
+def attn_sparse_fwd(q, k, v, heads, pivot_idx, query_window, key_window_times, *, want_lse=False, dropout=None):
     """Sparse TRAINING attention (mpu/sparse_transformer.py:675-725): q, k, v [b, s, heads*64] bf16 views,
-    pivot_idx int64 [b, n_piv].  Returns ctx [b, s, heads*64] bf16 (and lse [b, heads, s] fp32)."""
+    pivot_idx int64 [b, n_piv].  dropout: None or (p, seed, site) — dropout on the joint softmax probabilities.
+    Returns ctx [b, s, heads*64] bf16 (and lse [b, heads, s] fp32; and the keep-bit tensor when dropout is on)."""
     require_cuda(q, k, v, pivot_idx)
     b, s, h = q.shape
     n_piv = pivot_idx.shape[1]
@@ -188,6 +189,18 @@ def attn_sparse_fwd(q, k, v, heads, pivot_idx, query_window, key_window_times, *
     out = torch.empty((b, s, h), dtype=torch.bfloat16, device=q.device)
     lse = torch.empty((b, heads, s), dtype=torch.float32, device=q.device) if want_lse else None
     ws = torch.empty(lib().cv_attn_sparse_workspace_bytes(b, heads, 64, n_piv), dtype=torch.uint8, device=q.device)
+    dp, dseed, dsite = _drop3(dropout)
+    if dp > 0:
+        # keep bits in three regions (include/cogview_b200.h): band key-major, pivot key-major, query-major
+        words = lib().cv_attn_sparse_drop_mask_words(b, heads, s, n_piv, int(query_window), int(key_window_times))
+        mask = torch.empty(words, dtype=torch.int32, device=q.device)
+        rc = lib().cv_attn_sparse_dropout_fwd(ptr(q), q.stride(1), q.stride(0), ptr(k), k.stride(1), k.stride(0), ptr(v),
+                                              v.stride(1), v.stride(0), ptr(pivot_idx), ptr(out), out.stride(1),
+                                              out.stride(0), ptr(lse), ptr(ws), b, heads, 64, s, n_piv,
+                                              int(query_window), int(key_window_times), dp, dseed, dsite, ptr(mask),
+                                              stream_ptr())
+        check(rc, "cv_attn_sparse_dropout_fwd")
+        return (out, lse, mask) if want_lse else (out, mask)
     rc = lib().cv_attn_sparse_fwd(ptr(q), q.stride(1), q.stride(0), ptr(k), k.stride(1), k.stride(0), ptr(v), v.stride(1),
                                   v.stride(0), ptr(pivot_idx), ptr(out), out.stride(1), out.stride(0), ptr(lse), ptr(ws),
                                   b, heads, 64, s, n_piv, int(query_window), int(key_window_times), stream_ptr())
@@ -195,8 +208,10 @@ def attn_sparse_fwd(q, k, v, heads, pivot_idx, query_window, key_window_times, *
     return (out, lse) if want_lse else out
 
 
-def attn_sparse_bwd(q, k, v, out, d_out, lse, heads, pivot_idx, query_window, key_window_times):
-    """Backward of attn_sparse_fwd.  Returns dqkv [b, s, 3*heads*64] bf16 (dQ | dK | dV)."""
+def attn_sparse_bwd(q, k, v, out, d_out, lse, heads, pivot_idx, query_window, key_window_times, *, dropout_p=0.0,
+                    drop_mask=None):
+    """Backward of attn_sparse_fwd (dropout_p / drop_mask: the p and keep-bit tensor of a forward with dropout).
+    Returns dqkv [b, s, 3*heads*64] bf16 (dQ | dK | dV)."""
     require_cuda(q, k, v, out, d_out, lse, pivot_idx)
     b, s, h = q.shape
     n_piv = pivot_idx.shape[1]
@@ -205,6 +220,13 @@ def attn_sparse_bwd(q, k, v, out, d_out, lse, heads, pivot_idx, query_window, ke
     dqkv = torch.empty((b, s, 3 * h), dtype=torch.bfloat16, device=q.device)
     ws = torch.empty(lib().cv_attn_sparse_bwd_workspace_bytes(b, heads, 64, s, n_piv), dtype=torch.uint8,
                      device=q.device)
+    if dropout_p > 0:
+        rc = lib().cv_attn_sparse_dropout_bwd(ptr(q), q.stride(1), q.stride(0), ptr(k), k.stride(1), k.stride(0), ptr(v),
+                                              v.stride(1), v.stride(0), ptr(pivot_idx), ptr(out), ptr(d_out), ptr(lse),
+                                              ptr(dqkv), ptr(ws), b, heads, 64, s, n_piv, int(query_window),
+                                              int(key_window_times), float(dropout_p), ptr(drop_mask), stream_ptr())
+        check(rc, "cv_attn_sparse_dropout_bwd")
+        return dqkv
     rc = lib().cv_attn_sparse_bwd(ptr(q), q.stride(1), q.stride(0), ptr(k), k.stride(1), k.stride(0), ptr(v), v.stride(1),
                                   v.stride(0), ptr(pivot_idx), ptr(out), ptr(d_out), ptr(lse), ptr(dqkv), ptr(ws), b,
                                   heads, 64, s, n_piv, int(query_window), int(key_window_times), stream_ptr())

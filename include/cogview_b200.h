@@ -151,7 +151,22 @@ int cv_colsum_bf16(const void* dy, int64_t ld, void* out, float* workspace, int 
  * masked entries carry exactly -10000 as in the reference.  q / k / v: [b, s, heads*64] bf16 views as for cv_attn_fwd;
  * pivot_idx: int64 [b, n_piv] (distinct positions per sequence, mpu/sparse_transformer.py:557-565); s % w == 0.
  * The backward runs the band pass and the pivot pass with the joint lse / delta, scatters the pivot dK / dV back and
- * writes dqkv [b, s, 3*heads*64] (dQ | dK | dV).  Attention-probability dropout is not available in this mode.
+ * writes dqkv [b, s, 3*heads*64] (dQ | dK | dV).
+ *
+ * cv_attn_sparse_dropout_fwd / _bwd add dropout on the joint softmax probabilities (mpu/sparse_transformer.py:718-720),
+ * with the generator of cv_attn_fwd: one Philox4x32-10 call per (query, 128-key tile) seeds four 32-step LCG streams,
+ * keep iff state >= p * 2^32.  Band tiles use their key-tile index as counter, pivot tile t uses ceil(s/128) + t, so
+ * pivot slots and band keys never share a decision.  Row sum and lse stay undropped; the output is scaled by 1/(1-p).
+ * drop_mask: uint32 buffer of cv_attn_sparse_drop_mask_words() words in three regions (nqb = ceil(s/128),
+ * npt = ceil(n_piv/128), T = the longest band + pivot tile list of any 128-query block):
+ *   [0] band key-major  [b, heads, nqb*128 (key), nqb, 4]: bit i of word w of (key, query block qb) is query
+ *       qb*128 + 32w + i — the layout of cv_attn_fwd's region [0];
+ *   [1] pivot key-major [b, heads, npt*128 (pivot slot), nqb, 4], same bit order;
+ *   [2] query-major     [b, heads, nqb*128 (query), T, 4]: entry j is the j-th tile the query's block visits (band
+ *       tiles ceil(band_start(qb*128)/128) .. qb, then, if band_start of the block's last query > 0, all npt pivot
+ *       tiles); bit i of word w is key (or pivot slot) 32w + i of that tile.
+ * Tiles a block never visits are left unwritten.  The backward reads regions [0] and [1] (pass the same pointer).
+ * cv_attn_sparse_fwd / _bwd are these with dropout_p = 0.
  * ---------------------------------------------------------------------------------------------- */
 int64_t cv_attn_sparse_workspace_bytes(int b, int heads, int head_dim, int n_piv);
 int cv_attn_sparse_fwd(const void* q, int64_t ldq, int64_t bsq, const void* k, int64_t ldk, int64_t bsk, const void* v,
@@ -163,6 +178,17 @@ int cv_attn_sparse_bwd(const void* q, int64_t ldq, int64_t bsq, const void* k, i
                        int64_t ldv, int64_t bsv, const int64_t* pivot_idx, const void* out, const void* d_out,
                        const float* lse, void* dqkv, void* workspace, int b, int heads, int head_dim, int s, int n_piv,
                        int query_window, int key_window_times, void* stream);
+int64_t cv_attn_sparse_drop_mask_words(int b, int heads, int s, int n_piv, int query_window, int key_window_times);
+int cv_attn_sparse_dropout_fwd(const void* q, int64_t ldq, int64_t bsq, const void* k, int64_t ldk, int64_t bsk,
+                               const void* v, int64_t ldv, int64_t bsv, const int64_t* pivot_idx, void* out,
+                               int64_t ldo, int64_t bso, float* lse, void* workspace, int b, int heads, int head_dim,
+                               int s, int n_piv, int query_window, int key_window_times, float dropout_p,
+                               uint64_t seed, uint32_t site, uint32_t* drop_mask, void* stream);
+int cv_attn_sparse_dropout_bwd(const void* q, int64_t ldq, int64_t bsq, const void* k, int64_t ldk, int64_t bsk,
+                               const void* v, int64_t ldv, int64_t bsv, const int64_t* pivot_idx, const void* out,
+                               const void* d_out, const float* lse, void* dqkv, void* workspace, int b, int heads,
+                               int head_dim, int s, int n_piv, int query_window, int key_window_times, float dropout_p,
+                               const uint32_t* drop_mask, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Decode (one new token per sequence): HBM-bound weight streaming, CUDA cores.
